@@ -2,6 +2,7 @@
 """Benchmark of the ASR train-step hot path (BASELINE.json metric: utterances/sec, ~12 s @ 16 kHz synthetic).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfgB|cfgC|cfgD] [--impl b200|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one full train step over one synthetic batch: fused front end (STFT+mel+log, delta, CMVN) -> encoder ->
 CTC (+ attention decoder + CE) -> backward -> [NCCL grad all-reduce] -> grad-norm / clip / Adadelta.
@@ -62,7 +63,16 @@ def parse_args():
     ap.add_argument("--parity-workloads", default="auto",
                     help="comma list of workloads parity-checked at full size after the timed regions "
                          "(auto = the benchmarked one, plus cfgB,cfgC,cfgD on a default 1-GPU run)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy: loss, grad_norm, and a fixed "
+                         "sample of the updated parameters and of the gradient (params, grad), so that two builds can "
+                         "be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 train step")
+    return args
 
 
 T0 = time.time()
@@ -128,6 +138,25 @@ class ClockSampler:
                 pass
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons),
                 "samples": len(sm)}
+
+
+DUMP_SAMPLE = 4 << 20       # elements kept of each flat buffer: 2 x 16 MB of float32
+
+
+def step_outputs(step_fn, loss):
+    """What a caller of the train step holds after it, as float arrays: the loss it returned, the gradient norm, and
+    the model's flat parameter buffer (after the update) and gradient buffer.  A buffer larger than DUMP_SAMPLE
+    elements is cut to a fixed random sample of that many (seed 0, ascending indices)."""
+    import numpy as np
+    buf = step_fn.optimizer.buf
+    idx = None
+    if buf.total > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(buf.total, DUMP_SAMPLE, replace=False))
+        idx = torch.from_numpy(idx).to(buf.flat.device)
+    pick = (lambda t: t) if idx is None else (lambda t: t[idx])
+    return {"loss": np.array([loss], np.float32),
+            "grad_norm": step_fn.optimizer.grad_norm.detach().cpu().numpy().astype(np.float32),
+            "params": pick(buf.flat).cpu().numpy(), "grad": pick(buf.grad).cpu().numpy()}
 
 
 def build_cpu_reference(cfg, vocab, seed=0):
@@ -572,6 +601,7 @@ def main():
     if rank == 0:
         sampler.start()
     eager_ms, loss, launches = timed(step_resident, args.steps, profile=True)
+    dump = step_outputs(step_fn, loss) if args.dump_outputs else None
     summary = pkg.lib.TIMER.summary()
     launches_per_step = launches / args.steps
     log("eager timed region done: %.1f ms/step" % (eager_ms / args.steps))
@@ -593,9 +623,16 @@ def main():
         for _ in range(3):
             step_resident()
         ms, loss, _ = timed(step_resident, args.steps)
+        dump = step_outputs(step_fn, loss) if args.dump_outputs else None
     else:
         ms = eager_ms
     clocks = sampler.stop() if rank == 0 else None
+    if dump is not None and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+        log("outputs of the last timed step written to %s" % args.dump_outputs)
     log("timed region done: %.1f ms/step" % (ms / args.steps))
     value = gb * args.steps / (ms / 1000.0)
     e2e = None

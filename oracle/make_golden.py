@@ -1,12 +1,13 @@
 """Generate tests/golden/*.npz by RUNNING the unmodified reference (CPU) in the build container.
 
-    python -m oracle.make_golden            # from the repo root; needs /root/reference
+    B200ASR_REFERENCE=<checkout of the original project> python -m oracle.make_golden     # from the repo root
 
 The vectors pin the oracle (oracle_np.py, ref_port.py) and are the committed authority the GPU parity tests compare
 against on the GPU box, where /root/reference does not exist.  Everything is seeded; sizes are tiny on purpose.
 """
 import os
 import sys
+import zlib
 
 import numpy as np
 import torch
@@ -14,6 +15,8 @@ import torch
 from . import ref_shim
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+GRAD_FULL_MAX = 32768       # gradients with more elements are stored as a sample of GRAD_SAMPLE of them (files < 1 MB)
+GRAD_SAMPLE = 8192
 
 AUDIO_CFG = dict(feat_type="fbank", feat_dim=40, frame_length=25, frame_shift=10, dither=0, apply_cmvn=True,
                  delta_order=2, delta_window_size=2)
@@ -130,13 +133,23 @@ def golden_model(kind, seed, B, T, D, V, Lmax):
     out["total_loss"] = total.detach().numpy()
     gn = torch.nn.utils.clip_grad_norm_(model.parameters(), 5.0)
     out["grad_norm"] = np.float32(gn)
+    # The initial weights are the seeded init_adadelta initialisation, which the package's ASR reproduces bit for bit:
+    # keep the seed and each tensor's shape and CRC-32 instead of the values (tests/conftest.py: golden_params).
+    out["seed"], out["vocab"] = np.int64(seed), np.int64(V)
     for k, v in model.state_dict().items():
-        out["sd." + k] = v.numpy()
+        out["sd_shape." + k] = np.asarray(v.shape, np.int64)
+        out["sd_crc32." + k] = np.int64(zlib.crc32(np.ascontiguousarray(v.numpy()).tobytes()))
+    rng = np.random.default_rng(seed)
     for k, p in model.named_parameters():
         if p.grad is not None:
             # clip_grad_norm_ scaled the grads in place: undo so the vectors hold the raw gradients
             coef = min(1.0, 5.0 / (float(gn) + 1e-6))
-            out["grad." + k] = (p.grad / coef).numpy()
+            grad = (p.grad / coef).numpy()
+            if grad.size > GRAD_FULL_MAX:       # large gradients: a fixed random sample of their elements
+                idx = np.sort(rng.choice(grad.size, GRAD_SAMPLE, replace=False)).astype(np.int32)
+                out["grad_idx." + k] = idx
+                grad = grad.reshape(-1)[idx]
+            out["grad." + k] = grad
     # greedy inference outputs as well (teacher=None, argmax feedback), src/asr.py:137-142
     if att_out is not None:
         model.eval()

@@ -5,7 +5,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from conftest import load_golden, rel_err
+from conftest import golden_grad, golden_params, load_golden, rel_err
 from oracle.make_golden import tiny_model_cfg
 
 pytestmark = pytest.mark.gpu
@@ -15,12 +15,8 @@ DEV = "cuda"
 def _build(pkg, g, kind):
     cfg = tiny_model_cfg(kind)
     D = g["feat"].shape[-1]
-    V = g["sd.ctc_layer.weight"].shape[0] if "sd.ctc_layer.weight" in g else g["sd.pre_embed.weight"].shape[0]
-    model = pkg.ASR(D, V, True, **cfg)
-    sd = {k[3:]: torch.from_numpy(v) for k, v in g.items() if k.startswith("sd.")}
-    assert set(sd.keys()) == set(model.state_dict().keys())              # identical state_dict contract
-    for k, v in model.state_dict().items():
-        assert tuple(v.shape) == tuple(sd[k].shape), k
+    model = pkg.ASR(D, int(g["vocab"]), True, **cfg)
+    sd = golden_params(g, kind)                                        # checks the state_dict contract as well
     model.load_state_dict(sd)
     return model.to(DEV), cfg
 
@@ -63,11 +59,10 @@ def test_train_step_matches_reference(pkg, kind):
     total.backward()
     sq = 0.0
     for k, p in model.named_parameters():
-        key = "grad." + k
-        if key in g:
-            ref = g[key]
+        if "grad." + k in g:
+            mine, ref = golden_grad(g, k, p.grad.cpu().numpy())
             scale = max(float(np.abs(ref).max()), 1e-4)
-            assert float(np.abs(p.grad.cpu().numpy() - ref).max()) < 2e-4 * scale, k
+            assert float(np.abs(mine - ref).max()) < 2e-4 * scale, k
             sq += float((p.grad.double() ** 2).sum())
     assert abs(np.sqrt(sq) - float(g["grad_norm"])) < 1e-4 * float(g["grad_norm"])
 

@@ -92,7 +92,7 @@ def test_state_dict_contract_matches_reference_goldens(pkg):
         g = load_golden("model_%s.npz" % kind)
         cfg = tiny_model_cfg(kind)
         model = pkg.ASR(8, 12, True, **cfg)
-        ref_keys = {k[3:]: v.shape for k, v in g.items() if k.startswith("sd.")}
+        ref_keys = {k[len("sd_shape."):]: v for k, v in g.items() if k.startswith("sd_shape.")}
         mine = {k: tuple(v.shape) for k, v in model.state_dict().items()}
         assert mine == {k: tuple(s) for k, s in ref_keys.items()}
         assert model.enable_ctc == (cfg["ctc_weight"] > 0) and model.enable_att == (cfg["ctc_weight"] != 1)

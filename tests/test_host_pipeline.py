@@ -8,7 +8,7 @@ import pytest
 import torch
 import torch.multiprocessing as mp
 
-from conftest import GOLDEN, ROOT, load_golden
+from conftest import GOLDEN, ROOT, golden_params, load_golden
 
 
 def test_character_encoder_known_answers(pkg):
@@ -82,7 +82,7 @@ def _dp_worker(rank, world, port, out):
     dp = pkg.dist.DataParallel(backend="gloo")
     g = dict(np.load(os.path.join(GOLDEN, "model_hybrid.npz")))
     cfg = tiny_model_cfg("hybrid")
-    P = {k[3:]: torch.from_numpy(v).clone().requires_grad_(True) for k, v in g.items() if k.startswith("sd.")}
+    P = {k: v.requires_grad_(True) for k, v in golden_params(g, "hybrid").items()}
     feat, flen, txt = torch.from_numpy(g["feat"]), torch.from_numpy(g["feat_len"]), torch.from_numpy(g["txt"])
     B = feat.shape[0]
     ntok = float((txt != 0).sum())

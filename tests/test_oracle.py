@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import load_golden, rel_err
+from conftest import golden_grad, golden_params, load_golden, rel_err
 from oracle import oracle_np as onp
 from oracle import ref_port
 from oracle.make_golden import AUDIO_CFG, tiny_model_cfg
@@ -84,14 +84,10 @@ def test_ctc_np_matches_aten_cases():
 
 
 # ------------------------------------------------------------------------------------------- model
-def _P(g):
-    return {k[3:]: torch.from_numpy(v) for k, v in g.items() if k.startswith("sd.")}
-
-
 @pytest.mark.parametrize("kind", ["ctc", "hybrid", "cnn", "att", "vgg"])
 def test_ref_port_matches_reference_model(kind):
     g = load_golden("model_%s.npz" % kind)
-    P = {k: v.clone().requires_grad_(True) for k, v in _P(g).items()}
+    P = {k: v.requires_grad_(True) for k, v in golden_params(g, kind).items()}
     cfg = tiny_model_cfg(kind)
     res = ref_port.forward_losses(P, cfg, torch.from_numpy(g["feat"]), torch.from_numpy(g["feat_len"]),
                                   torch.from_numpy(g["txt"]))
@@ -109,25 +105,24 @@ def test_ref_port_matches_reference_model(kind):
     assert abs(float(res["total_loss"]) - float(g["total_loss"])) < tol
     for k, p in P.items():
         if ("grad." + k) in g:
-            assert rel_err(p.grad.numpy(), g["grad." + k], floor=1e-4) < 1e-3, k
+            assert rel_err(*golden_grad(g, k, p.grad.numpy()), floor=1e-4) < 1e-3, k
     norm, _ = ref_port.grad_norm_clip([p.grad for p in P.values() if p.grad is not None])
     assert abs(float(norm) - float(g["grad_norm"])) < tol
 
 
 def test_lstm_np_matches_reference_layer():
     g = load_golden("model_ctc.npz")
-    P = {k: v.numpy() for k, v in _P(g).items()}
+    Pt = golden_params(g, "ctc")
     pre = "encoder.layers.0.layer."
-    params = {k[len(pre):]: v for k, v in P.items() if k.startswith(pre)}
+    params = {k[len(pre):]: v.numpy() for k, v in Pt.items() if k.startswith(pre)}
     out = onp.bilstm(g["feat"], params)
-    Pt = _P(g)
     ref, _ = ref_port._lstm(Pt, pre, torch.from_numpy(g["feat"]), True)
     assert np.max(np.abs(out - ref.numpy())) < 1e-6      # fp64 restatement vs ATen fp32
 
 
 def test_attention_step_np_matches_port():
     g = load_golden("model_hybrid.npz")
-    P = _P(g)
+    P = golden_params(g, "hybrid")
     cfg = tiny_model_cfg("hybrid")
     enc, enc_len = ref_port.encoder(P, cfg["encoder"], torch.from_numpy(g["feat"]), torch.from_numpy(g["feat_len"]))
     key = torch.tanh(torch.nn.functional.linear(enc, P["attention.proj_k.weight"], P["attention.proj_k.bias"]))

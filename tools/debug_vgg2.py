@@ -2,13 +2,16 @@
 import os, sys, numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+from conftest import golden_params
 g = dict(np.load(os.path.join(ROOT, "tests", "golden", "model_vgg.npz")))
+P = golden_params(g, "vgg")
 def build():
     c0, c1 = 64, 128
     ext = torch.nn.Sequential(
         torch.nn.Conv2d(1, c0, 3, 1, 1), torch.nn.ReLU(), torch.nn.Conv2d(c0, c0, 3, 1, 1), torch.nn.ReLU(), torch.nn.MaxPool2d(2, 2),
         torch.nn.Conv2d(c0, c1, 3, 1, 1), torch.nn.ReLU(), torch.nn.Conv2d(c1, c1, 3, 1, 1), torch.nn.ReLU(), torch.nn.MaxPool2d(2, 2))
-    sd = {k[len("sd.encoder.layers.0.extractor."):]: torch.from_numpy(v) for k, v in g.items() if k.startswith("sd.encoder.layers.0.extractor.")}
+    sd = {k[len("encoder.layers.0.extractor."):]: v for k, v in P.items() if k.startswith("encoder.layers.0.extractor.")}
     ext.load_state_dict(sd)
     return ext
 feat = torch.from_numpy(g["feat"])
