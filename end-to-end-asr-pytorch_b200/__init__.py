@@ -5,8 +5,8 @@ The directory name follows the reference repository; import it with
 (or `import b200asr`, the alias module at the repo root).  Layout:
     csrc/      hand-written CUDA kernels + the C ABI (include/b200asr.h) -> libb200asr.so
     lib.py     ctypes binding;  ops.py  autograd wrappers
-    audio.py / module.py / asr.py / optim.py / solver.py / train_asr.py / test_asr.py / data.py / text.py
-               host-side mirror of the reference's src/ + bin/train_asr.py API (same names and signatures)
+    audio.py / module.py / asr.py / lm.py / optim.py / solver.py / train_asr.py / test_asr.py / train_lm.py / data.py /
+    text.py    host-side mirror of the reference's src/ + bin/train_{asr,lm}.py API (same names and signatures)
 """
 from . import lib
 from . import ops
@@ -14,7 +14,7 @@ from .lib import B200AsrError, load as load_library
 from .audio import create_transform, FbankFrontEnd
 from .asr import ASR, Encoder, Decoder, Attention
 from .ops import CTCLoss
-from . import audio, module, asr, optim, dist, synthetic, trainer, util, text, data, corpus, option, solver, train_asr, test_asr, ctc
+from . import audio, module, asr, optim, dist, synthetic, trainer, util, text, data, corpus, option, solver, train_asr, test_asr, ctc, lm, train_lm
 from .optim import Optimizer
 from .trainer import TrainStep
 

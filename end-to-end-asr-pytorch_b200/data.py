@@ -156,3 +156,66 @@ def _data_msg(name, path, train_split, tr_set, dev_split, dv_set, batch_size, bu
             "           | Train sets = {}\t| Number of utts = {}".format(train_split, tr_set),
             "           | Dev sets = {}\t| Number of utts = {}".format(dev_split, dv_set),
             "           | Batch size = {}\t\t| Bucketing = {}".format(batch_size, bucketing)]
+
+
+# ---- text data of the RNN language model (the reference's src/data.py:46-61,107-126,159-177)--------------------
+def collect_text_batch(batch, mode):
+    """[[tokens, ...]] (one bucket) or [tokens, ...] -> txt [B, L] int64, zero padded; in train mode the batch is
+    halved when its first sequence is longer than HALF_BATCHSIZE_TEXT_LEN tokens."""
+    if type(batch[0][0]) is list:
+        batch = batch[0]
+    if len(batch[0]) > HALF_BATCHSIZE_TEXT_LEN and mode == "train":
+        batch = batch[:len(batch) // 2]
+    return pad_sequence([torch.LongTensor(b) for b in batch], batch_first=True)
+
+
+class SyntheticTextDataset(Dataset):
+    """Seeded text buckets for runs without a corpus: item i is a bucket of `batch_size` token lists, longest first,
+    with lengths ~ U[min_len, max_len] (<eos> included), ids in [2, V) and <eos> = 1 last."""
+
+    def __init__(self, vocab_size, batch_size, n_batches, seed, min_len=20, max_len=60):
+        self.vocab_size, self.batch_size, self.n_batches, self.seed = vocab_size, batch_size, n_batches, seed
+        self.min_len, self.max_len = min_len, max_len
+
+    def __len__(self):
+        return self.n_batches
+
+    def __getitem__(self, i):
+        g = torch.Generator().manual_seed(self.seed + i)
+        lens = torch.sort(torch.randint(self.min_len, self.max_len + 1, (self.batch_size,), generator=g),
+                          descending=True)[0]
+        return [torch.randint(2, self.vocab_size, (int(n) - 1,), generator=g).tolist() + [1] for n in lens]
+
+
+def create_textset(tokenizer, train_split, dev_split, name, path, bucketing, batch_size, **extra):
+    """(tr_set, dv_set, tr_loader_bs, dv_loader_bs, msg) as src/data.py:107-126; the dev set is never bucketed."""
+    if name.lower() == "synthetic":
+        tr_set = SyntheticTextDataset(tokenizer.vocab_size, batch_size, extra.get("n_batches", 64), 0,
+                                      extra.get("min_len", 20), extra.get("max_len", 60))
+        dv_set = SyntheticTextDataset(tokenizer.vocab_size, batch_size, 2, 10 ** 6,
+                                      extra.get("min_len", 20), extra.get("max_len", 60))
+        msg = _data_msg(name, path, str(train_split), len(tr_set), str(dev_split), len(dv_set), batch_size, True)
+        return tr_set, dv_set, 1, 1, msg
+    if name.lower() != "librispeech":
+        raise NotImplementedError(name)
+    from .corpus import LibriTextDataset
+    bucket_size = batch_size if bucketing else 1
+    tr_loader_bs = 1 if bucketing else batch_size
+    dv_set = LibriTextDataset(path, dev_split, tokenizer, 1)
+    tr_set = LibriTextDataset(path, train_split, tokenizer, bucket_size)
+    msg = _data_msg(name, path, str(train_split), len(tr_set), str(dev_split), len(dv_set), batch_size, bucketing)
+    return tr_set, dv_set, tr_loader_bs, batch_size, msg
+
+
+def load_textset(n_jobs, use_gpu, pin_memory, corpus, text):
+    """(tr_loader, dv_loader, vocab_size, tokenizer, msg) as src/data.py:159-177.  The text lives in host memory, so
+    the loaders use no worker processes (n_jobs is accepted for the reference's signature)."""
+    synthetic = corpus["name"].lower() == "synthetic"
+    tokenizer = _VocabOnly(corpus.get("vocab_size", 31)) if synthetic else load_text_encoder(**text)
+    tr_set, dv_set, tr_bs, dv_bs, msg = create_textset(tokenizer, **corpus)
+    tr_loader = DataLoader(tr_set, batch_size=tr_bs, shuffle=True, drop_last=True,
+                           collate_fn=partial(collect_text_batch, mode="train"), num_workers=0, pin_memory=use_gpu)
+    dv_loader = DataLoader(dv_set, batch_size=dv_bs, shuffle=False, drop_last=False,
+                           collate_fn=partial(collect_text_batch, mode="dev"), num_workers=0, pin_memory=pin_memory)
+    msg.append("I/O spec.  | Token type = {}\t| Vocab size = {}".format(tokenizer.token_type, tokenizer.vocab_size))
+    return tr_loader, dv_loader, tokenizer.vocab_size, tokenizer, msg

@@ -80,6 +80,8 @@ SIGNATURES = {
     "b200asr_gemm3x_nt_pre": (c_int, [_P, _P, c_longlong, c_longlong, c_int, _P, _P, c_longlong, c_longlong, c_int, _P, c_int,
                                       c_int, c_int, c_int, c_int, c_int, c_int, _P, c_size_t, _P]),
     "b200asr_split_tf32": (c_int, [_P, _P, _P, c_longlong, _P]),
+    "b200asr_embedding_fwd": (c_int, [_P, c_longlong, _P, c_longlong, c_int, _P, _P]),
+    "b200asr_embedding_bwd": (c_int, [_P, _P, c_longlong, _P, c_longlong, c_int, _P, c_int, _P]),
     "b200asr_grad_norm_scratch_bytes": (c_size_t, []),
     "b200asr_grad_norm": (c_int, [_P, c_longlong, _P, _P, _P]),
     "b200asr_adadelta_step": (c_int, [_P, _P, _P, _P, c_longlong, c_float, c_float, c_float, c_float, _P, c_float, _P]),

@@ -318,6 +318,54 @@ def _gemm_ops():
     return (Split, mm3) if GEMM_MODE in ("tf32x3", "umma") else (Plain, mm1)
 
 
+def _bilstm_forward(ctx, x, ndir, params):
+    """BiLSTMFn.forward; also returns the cell states cst [ndir, B, T, H] (saved for the backward, which reads them)."""
+    lib = L.load()
+    assert len(params) == 4 * ndir
+    Op, mm = _gemm_ops()
+    x = _f32c(x)
+    B, T, I = x.shape
+    H = params[1].shape[1]
+    dev = x.device
+    perm = gate_perm(H, dev)
+    umma = _use_umma(I)
+    xs = None if umma else Op(x.view(B * T, I))
+    gates = torch.empty((ndir, B, T, H, 4), device=dev, dtype=torch.float32)
+    w_ih_p, w_ih_lo = [], []
+    # the layer input enters the forward projection of both directions and both dW_ih products: split it once
+    x_lo = tf32_residual(x) if (umma and PRESPLIT_ACTIVATIONS) else None
+    for d in range(ndir):
+        w_ih, w_hh, b_ih, b_hh = params[4 * d:4 * d + 4]
+        wp = w_ih.detach().index_select(0, perm)
+        bp = (b_ih.detach() + b_hh.detach()).index_select(0, perm)
+        if umma:
+            wlo = tf32_residual(wp)            # once per step: shared by the forward product and the input gradient
+            gemm_tn(x.view(B * T, I), wp, bias=bp, out=gates[d].view(B * T, 4 * H), w_lo=wlo,
+                    a_lo=x_lo.view(B * T, I) if x_lo is not None else None)
+            w_ih_lo.append(wlo)
+        else:
+            mm(xs, Op(wp).t(), out=gates[d].view(B * T, 4 * H), bias=bp)
+        w_ih_p.append(wp)
+    del xs
+    w_hh = torch.stack([_f32c(params[4 * d + 1].detach()) for d in range(ndir)]).contiguous()
+    cst = torch.empty((ndir, B, T, H), device=dev, dtype=torch.float32)
+    out = torch.empty((B, T, ndir * H), device=dev, dtype=torch.float32)
+    ws_bytes = lib.b200asr_bilstm_workspace_bytes(B, T, H, ndir)
+    if ws_bytes == 0:
+        raise L.B200AsrError("bilstm: no feasible decomposition for B=%d H=%d (H must be a multiple of 16)" % (B, H))
+    ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
+    # algorithmic bytes (SURVEY.md 8(d)): per step and direction read Gx[t] (16BH) + write h,c (8BH); W_hh once
+    with L.timed("bilstm_fwd", ndir * (24 * B * H * T + 16 * H * H)):
+        L.check(lib.b200asr_bilstm_fwd(L.ptr(gates), L.ptr(w_hh), L.ptr(cst), L.ptr(out), B, T, H, ndir,
+                                       L.ptr(ws), ws_bytes, L.stream()), "bilstm_fwd")
+    ctx.ndir = ndir
+    ctx.dims = (B, T, I, H)
+    ctx.consumed = False
+    ctx.has_x_lo = x_lo is not None
+    ctx.save_for_backward(x, gates, cst, out, w_hh, *w_ih_p, *w_ih_lo, *([x_lo] if x_lo is not None else []))
+    return out, cst
+
+
 class BiLSTMFn(Function):
     """One (bi)directional LSTM layer over zero-padded frames, zero initial state (src/module.py:129-132).
 
@@ -328,50 +376,7 @@ class BiLSTMFn(Function):
 
     @staticmethod
     def forward(ctx, x, ndir, *params):
-        lib = L.load()
-        assert len(params) == 4 * ndir
-        Op, mm = _gemm_ops()
-        x = _f32c(x)
-        B, T, I = x.shape
-        H = params[1].shape[1]
-        dev = x.device
-        perm = gate_perm(H, dev)
-        umma = _use_umma(I)
-        xs = None if umma else Op(x.view(B * T, I))
-        gates = torch.empty((ndir, B, T, H, 4), device=dev, dtype=torch.float32)
-        w_ih_p, w_ih_lo = [], []
-        # the layer input enters the forward projection of both directions and both dW_ih products: split it once
-        x_lo = tf32_residual(x) if (umma and PRESPLIT_ACTIVATIONS) else None
-        for d in range(ndir):
-            w_ih, w_hh, b_ih, b_hh = params[4 * d:4 * d + 4]
-            wp = w_ih.detach().index_select(0, perm)
-            bp = (b_ih.detach() + b_hh.detach()).index_select(0, perm)
-            if umma:
-                wlo = tf32_residual(wp)            # once per step: shared by the forward product and the input gradient
-                gemm_tn(x.view(B * T, I), wp, bias=bp, out=gates[d].view(B * T, 4 * H), w_lo=wlo,
-                        a_lo=x_lo.view(B * T, I) if x_lo is not None else None)
-                w_ih_lo.append(wlo)
-            else:
-                mm(xs, Op(wp).t(), out=gates[d].view(B * T, 4 * H), bias=bp)
-            w_ih_p.append(wp)
-        del xs
-        w_hh = torch.stack([_f32c(params[4 * d + 1].detach()) for d in range(ndir)]).contiguous()
-        cst = torch.empty((ndir, B, T, H), device=dev, dtype=torch.float32)
-        out = torch.empty((B, T, ndir * H), device=dev, dtype=torch.float32)
-        ws_bytes = lib.b200asr_bilstm_workspace_bytes(B, T, H, ndir)
-        if ws_bytes == 0:
-            raise L.B200AsrError("bilstm: no feasible decomposition for B=%d H=%d (H must be a multiple of 16)" % (B, H))
-        ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
-        # algorithmic bytes (SURVEY.md 8(d)): per step and direction read Gx[t] (16BH) + write h,c (8BH); W_hh once
-        with L.timed("bilstm_fwd", ndir * (24 * B * H * T + 16 * H * H)):
-            L.check(lib.b200asr_bilstm_fwd(L.ptr(gates), L.ptr(w_hh), L.ptr(cst), L.ptr(out), B, T, H, ndir,
-                                           L.ptr(ws), ws_bytes, L.stream()), "bilstm_fwd")
-        ctx.ndir = ndir
-        ctx.dims = (B, T, I, H)
-        ctx.consumed = False
-        ctx.has_x_lo = x_lo is not None
-        ctx.save_for_backward(x, gates, cst, out, w_hh, *w_ih_p, *w_ih_lo, *([x_lo] if x_lo is not None else []))
-        return out
+        return _bilstm_forward(ctx, x, ndir, params)[0]
 
     @staticmethod
     def backward(ctx, dout):
@@ -452,6 +457,91 @@ class BiLSTMFn(Function):
 
 def bilstm(x, lstm_params, ndir):
     return BiLSTMFn.apply(x, ndir, *lstm_params)
+
+
+class LSTMLastStateFn(Function):
+    """A unidirectional BiLSTMFn layer that also returns each row's cell state at its step last[b]: the c_n of a
+    packed nn.LSTM.  forward(x[B,T,I], last[B] int64 (device), w_ih, w_hh, b_ih, b_hh) -> (out[B,T,H], c_last[B,H]).
+    c_last is a copy that carries no gradient (the RNN-LM's training loss does not depend on it)."""
+
+    @staticmethod
+    def forward(ctx, x, last, *params):
+        out, cst = _bilstm_forward(ctx, x, 1, params)
+        c_last = cst[0, torch.arange(x.shape[0], device=x.device), last]
+        ctx.mark_non_differentiable(c_last)
+        return out, c_last
+
+    @staticmethod
+    def backward(ctx, dout, _dc_last):
+        dx, _, *grads = BiLSTMFn.backward(ctx, dout)
+        return (dx, None, *grads)
+
+
+def lstm_last_state(x, lstm_params, last):
+    return LSTMLastStateFn.apply(x, last, *lstm_params)
+
+
+# ----------------------------------------------------------------------------------------------------------
+class EmbeddingFn(Function):
+    """nn.Embedding without padding_idx (the RNN-LM's `emb`): row gather forward, deterministic segmented-sum weight
+    gradient (csrc/embedding.cu).  forward(ids int64 [...], weight [V,E]) -> [..., E]."""
+
+    @staticmethod
+    def forward(ctx, ids, weight):
+        lib = L.load()
+        w = _f32c(weight.detach())
+        V, E = w.shape
+        ids = _check_ids(ids, V)
+        out = torch.empty((ids.numel(), E), device=w.device, dtype=torch.float32)
+        with L.timed("embedding_fwd", 8 * ids.numel() + 8 * ids.numel() * E):
+            L.check(lib.b200asr_embedding_fwd(L.ptr(ids), ids.numel(), L.ptr(w), V, E, L.ptr(out), L.stream()),
+                    "embedding_fwd")
+        ctx.save_for_backward(ids)
+        ctx.V = V
+        return out.view(*ids.shape, E)
+
+    @staticmethod
+    def backward(ctx, dy):
+        (ids,) = ctx.saved_tensors
+        E = dy.shape[-1]
+        dw = torch.empty((ctx.V, E), device=dy.device, dtype=torch.float32)
+        embedding_backward(ids, dy, dw, accumulate=False, checked=True)
+        return None, dw
+
+
+def _check_ids(ids, V):
+    """int64, contiguous, on the device, every id in [0, V) - else B200AsrError (one 16-byte read-back)."""
+    if not ids.is_cuda:
+        raise L.B200AsrError("embedding: ids must be a CUDA tensor (got %s); there is no CPU fallback" % ids.device)
+    ids = ids.to(torch.int64).contiguous()
+    if ids.numel():
+        lo, hi = torch.stack(torch.aminmax(ids)).tolist()
+        if lo < 0 or hi >= V:
+            raise L.B200AsrError("embedding: ids must lie in [0, %d) (got min %d, max %d)" % (V, lo, hi))
+    return ids
+
+
+def embedding_backward(ids, dy, dw, accumulate=False, checked=False):
+    """dw[V,E] (= or +=) the weight gradient of the gather `table[ids]`, given its output gradient dy [..., E].  Rows
+    that receive no id are zeroed (or left as they are with accumulate).  The ids are stably sorted (torch.sort) so that every row
+    sums its contributions in ascending position: bit-identical across runs."""
+    lib = L.load()
+    V, E = dw.shape
+    assert dw.dtype == torch.float32 and dw.is_contiguous() and dy.shape[-1] == E
+    if not checked:
+        ids = _check_ids(ids, V)
+    flat = ids.reshape(-1)
+    dy = _f32c(dy).reshape(-1, E)
+    assert dy.shape[0] == flat.numel()
+    sorted_ids, order = torch.sort(flat, stable=True)
+    with L.timed("embedding_bwd", 4 * dy.numel() + 16 * flat.numel() + 4 * V * E * (2 if accumulate else 1)):
+        L.check(lib.b200asr_embedding_bwd(L.ptr(sorted_ids), L.ptr(order), flat.numel(), L.ptr(dy), V, E, L.ptr(dw),
+                                          int(bool(accumulate)), L.stream()), "embedding_bwd")
+    return dw
+
+
+def embedding(ids, weight):
+    return EmbeddingFn.apply(ids, weight)
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -1058,7 +1148,12 @@ class Linear3xFn(Function):
 
 def linear3x(x, layer):
     """Apply an nn.Linear through the 3xTF32 tensor-core path when the problem is large enough to matter."""
+    return dense3x(x, layer.weight, layer.bias)
+
+
+def dense3x(x, weight, bias=None):
+    """linear3x for a bare weight (e.g. a tied embedding matrix as the output projection)."""
     rows = x.numel() // x.shape[-1]
-    if x.is_cuda and rows * layer.in_features * layer.out_features >= (1 << 24):
-        return Linear3xFn.apply(x, layer.weight, layer.bias)
-    return torch.nn.functional.linear(x, layer.weight, layer.bias)
+    if x.is_cuda and rows * weight.shape[1] * weight.shape[0] >= (1 << 24):
+        return Linear3xFn.apply(x, weight, bias)
+    return torch.nn.functional.linear(x, weight, bias)

@@ -198,6 +198,19 @@ B200ASR_API int b200asr_ce_fwd_bwd(const float* logits, const long long* target,
                                    long long n_rows, int V, const float* grad_scale, float* row_loss,
                                    float* dlogits, b200asr_stream stream);
 
+/* ---- K17: token embedding (the RNN-LM's nn.Embedding, src/lm.py:17) forward and weight gradient --------------
+ * embedding_fwd: out[n, :] = W[ids[n], :] for n < N; W [V, E], out [N, E] row-major; id 0 is an ordinary row.
+ * embedding_bwd: dW[v, :] (accumulate ? += : =) sum of dY[n, :] over the n with ids[n] == v.  `sorted_ids` are the ids
+ *   sorted ascending with a STABLE sort and `order` the matching permutation (sorted_ids[i] == ids[order[i]]); each
+ *   row's sum runs in ascending position without atomics, so results are bit-reproducible.  Without `accumulate`
+ *   the rows that receive no id are zeroed.
+ * Ids outside [0, V) are never read through: the forward writes a zero row, the backward skips them (the caller is
+ * expected to reject them; ops.embedding does).                                                                     */
+B200ASR_API int b200asr_embedding_fwd(const long long* ids, long long N, const float* W, long long V, int E, float* out,
+                                      b200asr_stream stream);
+B200ASR_API int b200asr_embedding_bwd(const long long* sorted_ids, const long long* order, long long N, const float* dY,
+                                      long long V, int E, float* dW, int accumulate, b200asr_stream stream);
+
 /* ---- K16: gradient norm, clip and optimizer update on flat buffers (src/solver.py:84-89, src/optim.py) ----
  * grad_norm (device scalar) may be NULL (no clipping, no NaN skip); max_norm <= 0 disables clipping.          */
 B200ASR_API size_t b200asr_grad_norm_scratch_bytes(void);

@@ -3,8 +3,9 @@
 """Same command line as the reference's main.py (/root/reference/main.py:13-47), driving the B200-native Solver.
     python main.py --config config/b200/cfgB_ctc_char.yaml [--njobs 0] [--seed 0] [--load ckpt]
     torchrun --nproc-per-node 8 --master-addr 127.0.0.1 main.py --config ...      (data parallel, one process per GPU)
---test runs greedy decoding (decode.beam_size 1); --cpu hands the whole command line to the reference checkout
-(B200ASR_REFERENCE, default /root/reference) - this package has no CPU path; --lm is outside this hot path."""
+--test runs greedy decoding (decode.beam_size 1); --lm trains the RNN language model (config/b200/lm_example.yaml,
+one GPU) and takes precedence over --test as in the reference; --cpu hands the whole command line to the reference
+checkout (B200ASR_REFERENCE, default /root/reference) - this package has no CPU path."""
 import argparse
 import importlib
 import os
@@ -28,7 +29,7 @@ parser.add_argument("--cpu", action="store_true", help="(reference flag) use the
 parser.add_argument("--no-pin", action="store_true", help="Disable pin-memory for dataloader")
 parser.add_argument("--test", action="store_true", help="Test the model (greedy decoding, decode.beam_size: 1).")
 parser.add_argument("--no-msg", action="store_true", help="Hide all messages.")
-parser.add_argument("--lm", action="store_true", help="(reference flag) RNNLM training is outside this hot path")
+parser.add_argument("--lm", action="store_true", help="Train the RNN language model (single GPU).")
 parser.add_argument("--amp", action="store_true", help="(reference flag) unsupported")
 parser.add_argument("--reserve-gpu", default=0, type=float)
 parser.add_argument("--jit", action="store_true")
@@ -51,14 +52,16 @@ def main():
         os.chdir(ref)
         sys.argv[0] = os.path.join(ref, "main.py")
         return runpy.run_path(sys.argv[0], run_name="__main__")
-    if paras.lm or paras.cudnn_ctc:
-        raise SystemExit("--lm / --cudnn-ctc select reference paths outside the B200 hot path")
+    if paras.cudnn_ctc:
+        raise SystemExit("--cudnn-ctc selects a reference path outside the B200 hot path")
     config = yaml.load(open(paras.config, "r"), Loader=yaml.FullLoader)
     np.random.seed(paras.seed)
     torch.manual_seed(paras.seed)
     torch.cuda.manual_seed_all(paras.seed)
     pkg = importlib.import_module("end-to-end-asr-pytorch_b200")
-    if paras.test:          # greedy decoding (decode.beam_size: 1); beam search stays the reference's CPU path
+    if paras.lm:
+        solver = pkg.train_lm.Solver(config, paras, "train")
+    elif paras.test:        # greedy decoding (decode.beam_size: 1); beam search stays the reference's CPU path
         assert paras.load is None, "Load option is mutually exclusive to --test"
         solver = pkg.test_asr.Solver(config, paras, "test")
     else:
